@@ -34,7 +34,7 @@ NET_NAME = {"s3d": "S3D", "s3dg": "S3D-G", "r50": "R2D3D-50"}
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=_positive, default=8, help="timed training steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="coclr_b200", choices=["coclr_b200", "reference"])
     ap.add_argument("--precision", default="parity", choices=["parity", "mixed", "fast"])
@@ -56,7 +56,19 @@ def parse():
     ap.add_argument("--breakdown", action="store_true", help="print the per-kernel time table of one step to stderr")
     ap.add_argument("--timeline", action="store_true",
                     help="per-phase CUDA-event timeline of one step (ms since step start, max over ranks) in the JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, logits, targets, queue, a fixed sample of the "
+                         "encoder_q parameters and gradient) as DIR/<name>.npy, rank 0 only; the inputs depend only on "
+                         "the arguments and the training step sums in a fixed order, so repeated runs write the same "
+                         "arrays and two builds can be compared output for output")
     return ap.parse_args()
+
+
+def _positive(v):
+    n = int(v)
+    if n < 1:
+        raise argparse.ArgumentTypeError("must be >= 1")
+    return n
 
 
 # ------------------------------------------------------------------------------------------------
@@ -144,7 +156,7 @@ def reference_arm(args):
     if rank != 0:
         return
     batch, sample_T = CPU_SAMPLE_BATCH, CPU_SAMPLE_T
-    steps = max(1, min(args.steps, 10))
+    steps = args.steps
     val, med = cpu_oracle_clips_per_s(batch, sample_T, CFG["img"], args.moco_k, steps, 1, args.net)
     line = {"impl": "reference", "metric": "clips/sec %s InfoNCE (32x128^2, K=%d)" % (NET_NAME[args.net], args.moco_k), "value": val, "unit": "clips/s",
             "n_gpus": args.gpus, "steps": steps, "warmup": 1, "ms_per_step": med * 1e3, "higher_is_better": True,
@@ -158,6 +170,24 @@ def reference_arm(args):
                                        "is pure Python and cannot travel to the GPU box" % (steps, batch, sample_T, sample_T)},
             "e2e": {"value": val, "unit": "clips/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     emit(line)
+
+
+DUMP_MAX_ELEMS = 1 << 21     # per array: the six arrays of a dump stay under 64 MB whatever the shapes
+
+
+def dump_outputs(path, outputs):
+    """np.save every tensor of `outputs` (name -> tensor) as `path`/<name>.npy, float64 kept, everything else as float32.
+    A tensor of more than DUMP_MAX_ELEMS elements is flattened and sampled at sorted positions drawn from a fixed seed:
+    the same positions in every run with the same shapes."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        t = t.to("cpu", torch.float64 if t.dtype == torch.float64 else torch.float32)
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -392,20 +422,20 @@ def main():
     host_blocks = [torch.randn(nblk * B, 2, 3, T, HW, HW, generator=gen).pin_memory() for _ in range(2)]
     dev_blocks = [hb.to(dev) for hb in host_blocks]       # 2 x 403 MB > 126 MB L2: inputs never L2-resident
     vname = torch.randint(0, 997, (B,), device=dev)
-    loss_keep = [None, None]
+    loss_keep = [None, None, None]                         # loss, logits, labels (InfoNCE) / positive mask (CoCLR)
 
     def train_step(block):
         if coclr:
             import main_coclr
-            logits, mask = model(block[:B], block[B:], vname)
-            loss = main_coclr.multi_nce_loss(logits, mask)
+            logits, target = model(block[:B], block[B:], vname)
+            loss = main_coclr.multi_nce_loss(logits, target)
         else:
-            logits, labels = model(block)
-            loss = moco.nce_cross_entropy(logits, labels)
+            logits, target = model(block)
+            loss = moco.nce_cross_entropy(logits, target)
         opt.zero_grad()
         loss.backward()
         opt.step()
-        loss_keep[0], loss_keep[1] = loss, logits
+        loss_keep[0], loss_keep[1], loss_keep[2] = loss, logits, target
         return loss
 
     # ---- parity of this configuration, before anything is timed (all ranks take part; rank 0 runs the oracle) ----
@@ -443,6 +473,11 @@ def main():
     ms = float(t)
     final_loss = float(loss_keep[0].detach())
     value = 2.0 * B * world / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss_keep[0].reshape(1), "logits": loss_keep[1],
+                                         ("mask" if coclr else "labels"): loss_keep[2], "queue": model.queue,
+                                         "encoder_q_params": model.encoder_q.store.flat,
+                                         "encoder_q_grad": model.encoder_q.store.grad})
 
     # ---- end to end: pinned host inputs, H2D inside the timed region (prefetched), loss read back every step ----
     e2e = None

@@ -827,8 +827,9 @@ __global__ void __launch_bounds__(256) maxpool133s2_smem_kernel(const coclr_pool
   }
 }
 
-// scatter form of the backward: every output element adds its gradient to the one input element that won
-// (fp32 reductions in L2; a window overlaps up to 27 others, so this is ~27x less work than the gather form)
+// scatter form of the backward: every output element adds its gradient to the one input element that won.  Used only
+// for pools whose windows do not overlap, where every input receives at most one addend and the result does not
+// depend on the order of the fp32 reductions in L2.
 __global__ void __launch_bounds__(256) maxpool_bwd_scatter_kernel(const coclr_pool_t P) {
   const int C4 = P.C >> 2;
   const int khw = P.g.kh * P.g.kw;
@@ -853,6 +854,76 @@ __global__ void __launch_bounds__(256) maxpool_bwd_scatter_kernel(const coclr_po
       const int bb = rem / P.g.kw, cc = rem - bb * P.g.kw;
       const int ti = to * P.g.st - P.g.pt + a, yi = yo * P.g.sh - P.g.ph + bb, xi = xo * P.g.sw - P.g.pw + cc;
       atomicAdd(P.dx + ((((size_t)b * P.Ti + ti) * P.Hi + yi) * P.Wi + xi) * P.ldx + P.x_coff + c + k, dv[k]);
+    }
+  }
+}
+
+// gather form for the (3,3,3)/1 pool with padding 1 and equal input / output shapes (the SepInception branch-3 pools),
+// four inputs along x per thread: the 3 x 3 x 6 windows that can hold their maxima are read once for all four instead
+// of 27 times per input.  Each input's sum runs in a fixed window order.
+__global__ void __launch_bounds__(256) maxpool333_bwd_gather4_kernel(const coclr_pool_t P) {
+  const int C4 = P.C >> 2, W4 = P.Wi >> 2;
+  const long total = (long)P.B * P.Ti * P.Hi * W4 * C4;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+    const int cg = (int)(i % C4);
+    long r = i / C4;
+    const int x0 = (int)(r % W4) * 4; r /= W4;
+    const int yi = (int)(r % P.Hi); r /= P.Hi;
+    const int ti = (int)(r % P.Ti);
+    const int b = (int)(r / P.Ti);
+    const int c = cg * 4;
+    float acc[4][4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) acc[k][0] = acc[k][1] = acc[k][2] = acc[k][3] = 0.f;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      const int nt = ti + 1 - a;
+      if (nt < 0 || nt >= P.To) continue;
+#pragma unroll
+      for (int bb = 0; bb < 3; ++bb) {
+        const int ny = yi + 1 - bb;
+        if (ny < 0 || ny >= P.Ho) continue;
+        const size_t orow = (((size_t)b * P.To + nt) * P.Ho + ny) * P.Wo;
+#pragma unroll
+        for (int q = 0; q < 6; ++q) {
+          const int nx = x0 - 1 + q;
+          if (nx < 0 || nx >= P.Wo) continue;
+          const uchar4 id = *reinterpret_cast<const uchar4*>(P.idx + (orow + nx) * P.C + c);
+          const unsigned char taps[4] = {id.x, id.y, id.z, id.w};
+          // input x0 + k lies in column cc = k - q + 2 of window nx
+          bool hit = false;
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const int cc = k - q + 2;
+            if (cc < 0 || cc > 2) continue;
+            const int tap = (a * 3 + bb) * 3 + cc;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) hit |= taps[j] == tap;
+          }
+          if (!hit) continue;
+          const float4 d = ld4(P.dy + (orow + nx) * P.C + c);
+          const float dv[4] = {d.x, d.y, d.z, d.w};
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const int cc = k - q + 2;
+            if (cc < 0 || cc > 2) continue;
+            const int tap = (a * 3 + bb) * 3 + cc;
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+              if (taps[j] == tap) acc[k][j] += dv[j];
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      float* dp = P.dx + ((((size_t)b * P.Ti + ti) * P.Hi + yi) * P.Wi + x0 + k) * P.ldx + P.x_coff + c;
+      float4 v = make_float4(acc[k][0], acc[k][1], acc[k][2], acc[k][3]);
+      if (P.accumulate) {
+        const float4 old = ld4(dp);
+        v.x += old.x; v.y += old.y; v.z += old.z; v.w += old.w;
+      }
+      st4(dp, v);
     }
   }
 }
@@ -1264,9 +1335,12 @@ extern "C" int coclr_maxpool_fwd(const coclr_pool_t* p, coclr_stream_t stream) {
 }
 extern "C" int coclr_maxpool_bwd(const coclr_pool_t* p, coclr_stream_t stream) {
   if (!p || !p->dx || !p->dy || !p->idx || p->C % 4) return COCLR_E_ARG;
-  // scatter form whenever the destination can be zero-initialised with one memset (or already holds the other
-  // consumers' contributions); the gather kernel remains for strided destinations
-  if (p->accumulate || (p->ldx == p->C && p->x_coff == 0)) {
+  // scatter form when the windows do not overlap, so that every input element receives at most one addend, and the
+  // destination can be zero-initialised with one memset (or already holds the other consumers' contributions).
+  // Overlapping windows go to the gather kernel, which sums each input's windows in a fixed order: fp32 atomics from
+  // several windows would make the gradient, and every training step after it, differ from run to run.
+  const bool disjoint = p->g.kt <= p->g.st && p->g.kh <= p->g.sh && p->g.kw <= p->g.sw;
+  if (disjoint && (p->accumulate || (p->ldx == p->C && p->x_coff == 0))) {
     cudaStream_t s = (cudaStream_t)stream;
     if (!p->accumulate) {
       const size_t bytes = (size_t)p->B * p->Ti * p->Hi * p->Wi * p->C * sizeof(float);
@@ -1274,6 +1348,13 @@ extern "C" int coclr_maxpool_bwd(const coclr_pool_t* p, coclr_stream_t stream) {
     }
     const long tot_o = (long)p->B * p->To * p->Ho * p->Wo * (p->C / 4);
     maxpool_bwd_scatter_kernel<<<grid_for(tot_o, 256, 148 * 32), 256, 0, s>>>(*p);
+    return LAUNCH_OK();
+  }
+  const coclr_geom_t& g = p->g;
+  if (g.kt == 3 && g.kh == 3 && g.kw == 3 && g.st == 1 && g.sh == 1 && g.sw == 1 && g.pt == 1 && g.ph == 1 &&
+      g.pw == 1 && p->Wi % 4 == 0 && p->Wo == p->Wi && p->Ho == p->Hi && p->To == p->Ti) {
+    const long total4 = (long)p->B * p->Ti * p->Hi * (p->Wi / 4) * (p->C / 4);
+    maxpool333_bwd_gather4_kernel<<<grid_for(total4, 256, 148 * 32), 256, 0, (cudaStream_t)stream>>>(*p);
     return LAUNCH_OK();
   }
   const long total = (long)p->B * p->Ti * p->Hi * p->Wi * (p->C / 4);

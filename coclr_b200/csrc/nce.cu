@@ -165,23 +165,21 @@ __global__ void __launch_bounds__(256) nce_fwd_finish_kernel(const float* __rest
   }
 }
 
-// dq over a K slice, accumulated with fp32 atomics (dq zeroed by the caller path below)
-__global__ void __launch_bounds__(256) nce_bwd_slice_kernel(const float* __restrict__ dlogits, const float* __restrict__ k,
-                                                            const float* __restrict__ queue, float T, int D, int K,
-                                                            float* __restrict__ dq) {
-  __shared__ float sd[kNceSlice];
-  const int b = blockIdx.x, sl = blockIdx.y;
-  const int j0 = sl * kNceSlice, n = min(K - j0, kNceSlice);
-  for (int j = threadIdx.x; j < n; j += blockDim.x) sd[j] = dlogits[(long)b * (K + 1) + 1 + j0 + j];
-  __syncthreads();
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  const float d0 = dlogits[(long)b * (K + 1)];
-  for (int c = w; c < D; c += nw) {
-    float a = 0.f;
-    for (int j = lane; j < n; j += 32) a = fmaf(sd[j], __ldg(queue + (long)c * K + j0 + j), a);
-    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-    if (lane == 0) atomicAdd(dq + (long)b * D + c, (a + (sl == 0 ? d0 * k[(long)b * D + c] : 0.f)) / T);
-  }
+// dq for long queues: one warp per (row, channel) sums its whole dot product over the queue, channels spread over
+// blockIdx.y, so that the grid fills the SMs like the K slices of the forward.  Every dq element is written once, in a
+// fixed summation order: no atomics, and the same dq in every run.
+__global__ void __launch_bounds__(256) nce_bwd_cols_kernel(const float* __restrict__ dlogits, const float* __restrict__ k,
+                                                           const float* __restrict__ queue, float T, int D, int K,
+                                                           float* __restrict__ dq) {
+  const int b = blockIdx.x;
+  const int lane = threadIdx.x & 31, c = blockIdx.y * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (c >= D) return;
+  const float* drow = dlogits + (long)b * (K + 1);
+  const float* qrow = queue + (long)c * K;
+  float a = 0.f;
+  for (int j = lane; j < K; j += 32) a = fmaf(__ldg(drow + 1 + j), __ldg(qrow + j), a);
+  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+  if (lane == 0) dq[(long)b * D + c] = (a + drow[0] * k[(long)b * D + c]) / T;
 }
 
 }  // namespace coclr
@@ -206,9 +204,8 @@ extern "C" int coclr_nce_logits_bwd(const float* dlogits, const float* k, const 
                                     int K, float* dq, coclr_stream_t stream) {
   if (!dlogits || !k || !queue || !dq) return COCLR_E_ARG;
   if (K > 2 * kNceSlice) {
-    if (cudaMemsetAsync(dq, 0, sizeof(float) * (size_t)B * D, (cudaStream_t)stream) != cudaSuccess) return COCLR_E_LAUNCH;
-    const dim3 grid(B, (K + kNceSlice - 1) / kNceSlice);
-    nce_bwd_slice_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(dlogits, k, queue, T, D, K, dq);
+    const dim3 grid(B, (D + 7) / 8);
+    nce_bwd_cols_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(dlogits, k, queue, T, D, K, dq);
     return cudaGetLastError() == cudaSuccess ? COCLR_OK : COCLR_E_LAUNCH;
   }
   const size_t smem = (size_t)(K + 1) * sizeof(float);

@@ -1,10 +1,12 @@
-"""Generates tests/golden/infonce_cfg1.npz (and, with the argument `r50` / `s3dg`, infonce_r50.npz / infonce_s3dg.npz) by running the UNMODIFIED reference (TengdaHan/CoCLR at
-/root/reference, model/pretrain.py InfoNCE) on BASELINE.json config 1 (S3D, moco-k=128, bs=4,
+"""Generates tests/golden/infonce_cfg1.npz (and, with the argument `r50` / `s3dg`, infonce_r50.npz / infonce_s3dg.npz) by running the UNMODIFIED reference (TengdaHan/CoCLR,
+model/pretrain.py InfoNCE) on BASELINE.json config 1 (S3D, moco-k=128, bs=4,
 seq_len=8, 128x128, CPU) from the deterministic synthetic state of oracle.coclr_oracle.synth_state.
 
-Run in the build container only:  python tests/golden/make_golden.py
+Needs a checkout of the reference, named by the environment variable COCLR_REFERENCE:
+    COCLR_REFERENCE=/path/to/CoCLR python tests/golden/make_golden.py [r50|s3dg]
 The .npz stores reference outputs (logits, loss, updated queue/ptr, selected gradients and
-post-EMA key weights); inputs are regenerated from seeds by the tests.
+post-EMA key weights); inputs are regenerated from seeds by the tests.  The companion <name>_state.npz holds a
+sample of every entry of the reference model's state_dict after the step (see state_sample).
 """
 import os
 import sys
@@ -15,7 +17,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("COCLR_REFERENCE", "")
 
 
 def make_inputs(B=4, T=8, HW=128, seed=1234):  # noqa
@@ -52,6 +54,8 @@ def import_reference():
     """Import the UNMODIFIED reference's model.pretrain without clashing with this repo's own `model` /
     `backbone` packages (same top-level names by design: they are drop-ins)."""
     import importlib
+    if not os.path.isdir(os.path.join(REF, "model")):
+        raise SystemExit("set COCLR_REFERENCE to a checkout of the reference (TengdaHan/CoCLR)")
     clash = lambda k: k in ("model", "backbone") or k.startswith("model.") or k.startswith("backbone.")
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if clash(k)}
     sys.path.insert(0, REF)
@@ -65,6 +69,16 @@ def import_reference():
                 sys.modules.pop(k)
         sys.modules.update(saved)
     return mod
+
+
+def state_sample(sd, limit=128):
+    """Strided sample (compact) of every entry of a state_dict, packed as three arrays: the keys, the end offset of
+    each key's sample and all samples back to back as float32.  The post-step state of the reference is compared on
+    it; one array per key would cost more in archive headers than in data."""
+    keys = sorted(sd)
+    parts = [compact(sd[k].detach().float().numpy(), limit)[0].reshape(-1) for k in keys]
+    return {"state_keys": np.array(keys), "state_ends": np.cumsum([p.size for p in parts]),
+            "state_values": np.concatenate(parts).astype(np.float32)}
 
 
 GRAD_KEYS_R50 = ["encoder_q.0.conv1.weight", "encoder_q.0.bn1.weight", "encoder_q.0.layer1.0.conv2.weight",
@@ -133,12 +147,11 @@ def run_reference(K=128, B=4, T=8, ptr=16, threads=8, network="s3d", HW=128):
 
 if __name__ == "__main__":
     if "s3dg" in sys.argv[1:]:
-        out, _ = run_reference(network="s3dg", **S3DG_CFG)
-        np.savez_compressed(os.path.join(HERE, "infonce_s3dg.npz"), **out)
+        name, (out, model) = "infonce_s3dg", run_reference(network="s3dg", **S3DG_CFG)
     elif "r50" in sys.argv[1:]:
-        out, _ = run_reference(network="r50", **R50_CFG)
-        np.savez_compressed(os.path.join(HERE, "infonce_r50.npz"), **out)
+        name, (out, model) = "infonce_r50", run_reference(network="r50", **R50_CFG)
     else:
-        out, _ = run_reference()
-        np.savez_compressed(os.path.join(HERE, "infonce_cfg1.npz"), **out)
+        name, (out, model) = "infonce_cfg1", run_reference()
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    np.savez_compressed(os.path.join(HERE, name + "_state.npz"), **state_sample(model.state_dict()))
     print("loss", out["loss"], "logits[0,:4]", out["logits"][0, :4])

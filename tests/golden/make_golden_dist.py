@@ -2,8 +2,8 @@
 model.pretrain.InfoNCE (model/pretrain.py:98-190: shuffle-BN all-gather + rank-0 permutation broadcast, un-shuffle,
 global enqueue) wrapped in DistributedDataParallel as main_nce.py:172 does, one training forward/backward each.
 -> tests/golden/infonce_world2.npz (per-rank logits, replicated queue / pointer, DDP-averaged gradients).
-Pins oracle.infonce_forward's simulated multi-rank world.  Run in the build container only:
-    python tests/golden/make_golden_dist.py"""
+Pins oracle.infonce_forward's simulated multi-rank world.  Needs a checkout of the reference:
+    COCLR_REFERENCE=/path/to/CoCLR python tests/golden/make_golden_dist.py"""
 import os
 import sys
 

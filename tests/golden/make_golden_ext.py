@@ -1,5 +1,6 @@
 """Golden vectors for UberNCE and CoCLR from the UNMODIFIED reference (model/pretrain.py:193-418) on CPU:
-tests/golden/ubernce_cfg1.npz, tests/golden/coclr_cfg1.npz.  Run in the build container only."""
+tests/golden/ubernce_cfg1.npz, tests/golden/coclr_cfg1.npz.  Needs a checkout of the reference:
+    COCLR_REFERENCE=/path/to/CoCLR python tests/golden/make_golden_ext.py"""
 import os
 import sys
 

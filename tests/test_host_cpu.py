@@ -278,10 +278,13 @@ def test_space_to_depth_stem_is_the_same_convolution(stem):
     assert torch.equal(used, torch.ones_like(used))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/model"), reason="reference not mounted")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+
 def test_cli_accepts_every_reference_flag():
-    """Drop-in command line: every option of the reference's main_nce.py / main_coclr.py parses here, with the same
-    default for the options that shape the hot path."""
+    """Drop-in command line: every option of the reference's main_nce.py / main_coclr.py (tests/golden/reference_cli.json,
+    made by tests/golden/make_golden_cli.py) parses here, with the same default for the options that shape the hot path."""
+    import json
     import importlib.util
 
     def load(name):     # this repository's script by path (the reference has files of the same name)
@@ -290,19 +293,11 @@ def test_cli_accepts_every_reference_flag():
         spec.loader.exec_module(mod)
         return mod
     main_nce, main_coclr = load("main_nce"), load("main_coclr")
+    ref = json.load(open(os.path.join(GOLDEN, "reference_cli.json")))
+    assert len(ref["main_nce"]) > 30 and len(ref["main_coclr"]) > 30
 
-    def ref_flags(path):
-        out = {}
-        for m in re.finditer(r"add_argument\(([^)]*)\)", open(path).read()):
-            names = re.findall(r"'(-{1,2}[\w-]+)'", m.group(1))
-            takes_value = "store_true" not in m.group(1)
-            nargs2 = "nargs=2" in m.group(1)
-            for n in names:
-                out[n] = (takes_value, nargs2)
-        return out
-
-    for mod, path in ((main_nce, "/root/reference/main_nce.py"), (main_coclr, "/root/reference/main_coclr.py")):
-        for flag, (takes_value, nargs2) in ref_flags(path).items():
+    for mod, name in ((main_nce, "main_nce"), (main_coclr, "main_coclr")):
+        for flag, (takes_value, nargs2) in ref[name].items():
             argv = [flag] + ((["a", "b"] if nargs2 else ["1"]) if takes_value else [])
             try:
                 mod.parse_args(argv)
@@ -315,14 +310,13 @@ def test_cli_accepts_every_reference_flag():
     assert (c.topk, c.reverse, c.model, c.dataset) == (5, False, "coclr", "ucf101-2stream-2clip")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/model"), reason="reference not mounted")
 def test_training_losses_are_the_reference_formulas():
-    """The two mask losses of the training loops, executed from the reference's own source text (its scripts cannot be
-    imported: tensorboardX / lmdb are absent): multi_nce_loss (main_coclr.py:343-346) and the UberNCE loss lines
-    (main_nce.py:321-322) against main_coclr.multi_nce_loss / main_nce.multi_label_nce_loss, bit-for-bit."""
-    import ast
+    """The two mask losses of the training loops as the reference computes them (tests/golden/reference_losses.npz,
+    executed from the reference's own source text by tests/golden/make_golden_cli.py): multi_nce_loss
+    (main_coclr.py:343-346) and the UberNCE loss lines (main_nce.py:321-322) against main_coclr.multi_nce_loss /
+    main_nce.multi_label_nce_loss, bit-for-bit."""
     import importlib.util
-    import torch.nn.functional as F
+    import numpy as np
 
     def load(name):
         spec = importlib.util.spec_from_file_location("coclr_b200_cli2_" + name, os.path.join(ROOT, name + ".py"))
@@ -330,22 +324,12 @@ def test_training_losses_are_the_reference_formulas():
         spec.loader.exec_module(mod)
         return mod
     main_nce, main_coclr = load("main_nce"), load("main_coclr")
-    src = open("/root/reference/main_coclr.py").read()
-    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "multi_nce_loss"][0]
-    ns = {"torch": torch, "F": F}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), "ref_multi_nce_loss", "exec"), ns)
-    lines = open("/root/reference/main_nce.py").read().splitlines()
-    uber = [ln.strip() for ln in lines if ln.strip().startswith("loss = - (F.log_softmax(output, dim=1) * target)")]
-    assert len(uber) == 1
-    g = torch.Generator().manual_seed(9)
-    for _ in range(3):
-        logits = torch.randn(6, 1 + 40, generator=g) * 4
-        mask = torch.rand(6, 41, generator=g) < 0.15
-        mask[:, 0] = True
-        assert torch.equal(main_coclr.multi_nce_loss(logits, mask), ns["multi_nce_loss"](logits, mask))
-        env = {"F": F, "output": logits, "target": mask}
-        exec(uber[0], env)
-        assert torch.equal(main_nce.multi_label_nce_loss(logits, mask), env["loss"].mean())
+    ref = np.load(os.path.join(GOLDEN, "reference_losses.npz"))
+    assert len(ref["logits"]) == 3
+    for logits, mask, multi, uber in zip(ref["logits"], ref["mask"], ref["multi_nce_loss"], ref["ubernce_loss"]):
+        logits, mask = torch.from_numpy(logits), torch.from_numpy(mask)
+        assert torch.equal(main_coclr.multi_nce_loss(logits, mask), torch.tensor(multi))
+        assert torch.equal(main_nce.multi_label_nce_loss(logits, mask), torch.tensor(uber))
 
 
 def _load_cli(name):
@@ -384,11 +368,15 @@ def test_two_checkpoint_init_follows_reference(tmp_path):
     assert float(model.sampler[4].bias[0]) == 4.0
     assert torch.equal(model.encoder_k[0].Conv_2c.conv1.weight, a.encoder_q[0].Conv_2c.conv1.weight)
     assert torch.equal(model.queue, q0)                      # queues are always re-filled
-    # the reference's own merge, restated from its source text, gives the same key -> source mapping
-    ref_src = open("/root/reference/main_coclr.py").read() if os.path.exists("/root/reference/main_coclr.py") else ""
-    if ref_src:
-        assert "state_dict = {**first_dict, **second_dict}" in ref_src
-        assert "k = k.replace('encoder_q.', 'encoder_k.')" in ref_src and "k.replace('encoder_q.', 'sampler.')" in ref_src
+    # the reference's own merge gives the same key -> source mapping: tests/golden/reference_two_checkpoint.npz holds
+    # what it made of two checkpoints whose values name their own keys (tests/golden/make_golden_cli.py)
+    import numpy as np
+    ref = np.load(os.path.join(GOLDEN, "reference_two_checkpoint.npz"))
+    pa, pb = str(tmp_path / "a_names.pth.tar"), str(tmp_path / "b_names.pth.tar")
+    torch.save({"epoch": 7, "state_dict": {str(k): "first:" + str(k) for k in ref["first_keys"]}}, pa)
+    torch.save({"epoch": 9, "state_dict": {str(k): "second:" + str(k) for k in ref["second_keys"]}}, pb)
+    want = dict(zip(ref["merged_keys"].tolist(), ref["merged_values"].tolist()))
+    assert len(want) > 2000 and main_coclr.two_checkpoint_state([pa, pb]) == want
 
 
 def test_reference_adam_state_converts_to_flat(tmp_path):

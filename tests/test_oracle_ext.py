@@ -1,5 +1,6 @@
 """Pins the UberNCE / CoCLR restatements of the oracle against golden vectors from the unmodified reference
-(tests/golden/{ubernce,coclr}_cfg1*.npz) and, when the reference is mounted, against the reference itself."""
+(tests/golden/{ubernce,coclr}_cfg1*.npz): at fp32 level under any thread count, and bit-for-bit with the reference's
+thread count (8), which is how the golden vectors were made."""
 import os
 import sys
 
@@ -71,13 +72,12 @@ def test_coclr_oracle_matches_golden(full):
     assert np.array_equal(sd["queue_label"].numpy(), gold["queue_label"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/model"), reason="reference not mounted")
 def test_ext_bitwise_vs_reference():
     torch.set_num_threads(8)
-    ref_u = MX.run_ubernce()
+    ref_u = np.load(os.path.join(G, "ubernce_cfg1.npz"))
     _, logits, mask = oracle_ubernce()
     assert np.array_equal(logits.detach().numpy(), ref_u["logits"]) and np.array_equal(mask.numpy(), ref_u["mask"])
-    ref_c = MX.run_coclr(True)
+    ref_c = np.load(os.path.join(G, "coclr_cfg1.npz"))
     sd, logits, mask, _ = oracle_coclr(True)
     assert np.array_equal(logits.detach().numpy(), ref_c["logits"]) and np.array_equal(mask.numpy(), ref_c["mask"])
     assert np.array_equal(sd["queue_second"].numpy(), ref_c["queue_second"])
